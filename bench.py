@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rollout cost+gradient throughput, (seed x waypoint) evals/s.
 
-    python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl ours|reference]
+    python bench.py --gpus N --steps K --warmup W [--workload NAME] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the fused rollout kernel over one batch of synthetic joint configurations
 (= what one optimizer iteration's cost+gradient evaluation does, gradient_opt_core.py:445-480).
@@ -620,6 +620,8 @@ def main():
     ap.add_argument("--reference-design", type=int, default=1,
                     help="1 (N=1 only): time the reference's own kernels compiled for sm_100a, chained unfused from a CUDA graph "
                          "(scripts/bench_reference_design.py, separate process), under 'reference_design_gpu'")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the headline workload's outputs of its last timed step (the RolloutOutput arrays) as DIR/<name>.npy")
     ap.add_argument("--extra-workloads", default="franka_16384_esdf,franka_trajopt_32x32_esdf_swept,franka_mpc_1024x30_esdf_swept,franka_mpc_knots_1024x30_esdf_swept,franka_mpc_knots_inkernel_1024x30_esdf_swept,g1_29_8192_esdf,g1_43_8192_esdf,franka_mpc_1024x30_esdf_swept_dynamics_host,franka_mpc_1024x30_esdf_swept_dynamics,franka_mpc_knots_1024x30_esdf_swept_dynamics",
                     help="comma list, measured briefly on rank 0 at N=1 and reported under 'other_workloads'")
     args = ap.parse_args()
@@ -719,6 +721,8 @@ def main():
 
     wl, eng, q, ms_list, ms_warm = timed_run(args.workload, args.steps, args.warmup, preroll_s=0.5, warm_too=True)
     headline_kernel = last_kernel()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(eng.out, args.dump_outputs)             # before the e2e pipeline below reuses `eng`
     evals_per_step = wl["B"] * wl["H"]
     total_ms_max = max_over_ranks(float(sum(ms_list)))
     value = world * evals_per_step * args.steps / (total_ms_max * 1e-3)
@@ -901,6 +905,25 @@ def main():
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()
+
+
+def dump_outputs(out, directory, cap_bytes=64 << 20):
+    """Every array of a RolloutOutput as <directory>/<field>.npy: float32 as computed, integer fields as float64 (exact).
+    Above cap_bytes in all, every array keeps the same fixed seeded sample of its rows (leading axis), listed in rows.npy."""
+    import dataclasses
+    import torch
+    arrays = {f.name: getattr(out, f.name) for f in dataclasses.fields(out)}
+    arrays = {k: v.detach().cpu().numpy() for k, v in arrays.items() if torch.is_tensor(v)}
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in arrays.items()}
+    total = sum(v.nbytes for v in arrays.values())
+    if total > cap_bytes:
+        n = next(iter(arrays.values())).shape[0]
+        rows = np.sort(np.random.default_rng(0).choice(n, max(1, n * cap_bytes // total - 1), replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["rows"] = rows.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(directory, f"{k}.npy"), v)
 
 
 def reference_design_leg():

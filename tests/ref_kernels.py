@@ -1,16 +1,129 @@
-"""ctypes access to oracle/_ref/libcurobo_ref.so = the REFERENCE's own CUDA kernels compiled from
-/root/reference (test infrastructure only; see oracle/ref_kernels_launcher.cu)."""
+"""The REFERENCE's own CUDA kernels as the GPU tests compare with them (test infrastructure only).
+
+The tests read the kernels' outputs on each test's own inputs from tests/golden/reference_kernels_<group>.npz, recorded on a
+B200 so that the comparison needs nothing outside this repository.  The launchers below are ctypes access to
+oracle/_ref/libcurobo_ref.so, the reference's kernels compiled by `curobo_b200.build` from a checkout of the reference
+(oracle/ref_kernels_launcher.cu); they are what records the fixtures, from the repository root on a GPU:
+
+    CB200_RECORD_REFERENCE=<dir> python -m pytest -m gpu tests/test_gpu_parity.py tests/test_gpu_bspline.py \\
+        tests/test_gpu_optim.py tests/test_gpu_dynamics.py tests/test_gpu_zz_edt.py tests/test_gpu_zzz_center_of_mass.py
+    cp <dir>/reference_kernels_*.npz tests/golden/
+"""
 import ctypes as C
+import json
 import os
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PATH = os.path.join(ROOT, "oracle", "_ref", "libcurobo_ref.so")
+GOLDEN = os.path.join(ROOT, "tests", "golden")
+RECORD = os.environ.get("CB200_RECORD_REFERENCE")
+BUDGET = 1024        # elements kept per leading-axis length in a recorded case (whole entries of that axis)
 
 
 def available() -> bool:
+    """Whether the reference's kernels themselves are at hand (oracle/_ref, built where the reference's sources are)."""
     return os.path.exists(PATH)
+
+
+def comparing() -> bool:
+    """Whether tests compare with the reference's kernels: always, through the recorded outputs.  The emulated GPU suite
+    (tests/test_emulated_gpu_suite_cpu.py) turns it off: its host build of our kernels rounds differently from the device."""
+    return True
+
+
+def sample_rows(n, row_elems):
+    """Entries kept of a leading axis of length n whose entries hold row_elems elements (summed over the outputs sharing
+    the axis): all when they fit BUDGET, else the first, the last and a fixed seeded sample of the others."""
+    k = max(2, BUDGET // max(1, row_elems))
+    if n * row_elems <= BUDGET or k >= n:
+        return np.arange(n)
+    mid = np.random.default_rng(n).choice(np.arange(1, n - 1), k - 2, replace=False)
+    return np.sort(np.concatenate([[0, n - 1], mid])).astype(np.int64)
+
+
+class Recorded:
+    """r[i]: the reference's output i at its kept entries of the leading axis; r.at(i, a): the same entries of an array
+    `a` shaped like output i (ours, the oracle's); r.rows(i): their indices."""
+
+    def __init__(self, outs, rows, shapes):
+        self._outs, self._rows, self._shapes = outs, rows, shapes
+
+    def __len__(self):
+        return len(self._outs)
+
+    def __getitem__(self, i):
+        return self._outs[i]
+
+    def rows(self, i):
+        return self._rows[i]
+
+    def at(self, i, a):
+        assert tuple(np.shape(a)) == self._shapes[i], (np.shape(a), self._shapes[i])
+        return np.asarray(a)[self._rows[i]]
+
+
+def _read(path):
+    """{case name: [(full shape, kept rows, values) per output]} of one fixture file: one concatenated array per dtype
+    plus a JSON index (few archive members keep the file small)."""
+    with np.load(path) as g:
+        data = {k: g[k] for k in g.files}
+    recs = {}
+    for e in json.loads(str(data["index"])):
+        shape, rows = tuple(e["shape"]), np.asarray(e["rows"], np.int64)
+        v = data[e["dtype"]][e["offset"]:e["offset"] + e["count"]].reshape((len(rows),) + shape[1:])
+        recs.setdefault(e["name"], []).append((shape, rows, v))
+    return recs
+
+
+def _write(path, recs):
+    index, chunks, sizes = [], {}, {}
+    for name, outs in recs.items():
+        for shape, rows, v in outs:
+            dt = v.dtype.name
+            index.append({"name": name, "shape": list(shape), "rows": [int(r) for r in rows], "dtype": dt,
+                          "offset": sizes.get(dt, 0), "count": v.size})
+            chunks.setdefault(dt, []).append(v.reshape(-1))
+            sizes[dt] = sizes.get(dt, 0) + v.size
+    np.savez_compressed(path, index=np.array(json.dumps(index)), **{dt: np.concatenate(c) for dt, c in chunks.items()})
+
+
+_golden = {}
+
+
+def recorded(key, run, whole=False) -> Recorded:
+    """The reference's outputs for one test case: key = (group, name parts...); run() launches the reference's kernels on
+    the test's inputs and returns its outputs (a tensor or a sequence of them).  Outputs sharing a leading-axis length
+    keep the same entries of it (sample_rows); whole=True keeps every entry (sparse outputs, where a sample would hold
+    only zeros).  Replayed from tests/golden unless CB200_RECORD_REFERENCE names a directory: then run() is called and
+    its kept outputs are added to <dir>/reference_kernels_<group>.npz."""
+    group, name = key[0], "-".join(str(k) for k in key[1:])
+    fname = f"reference_kernels_{group}.npz"
+    if RECORD is None:
+        if group not in _golden:
+            _golden[group] = _read(os.path.join(GOLDEN, fname))
+        if name not in _golden[group]:
+            raise KeyError(f"no recorded reference output {name!r} in tests/golden/{fname}")
+        outs = _golden[group][name]
+        return Recorded([v for _, _, v in outs], [r for _, r, _ in outs], [s for s, _, _ in outs])
+    outs = run()
+    outs = [outs] if torch.is_tensor(outs) or isinstance(outs, np.ndarray) else list(outs)
+    torch.cuda.synchronize()
+    outs = [o.detach().cpu().numpy() if torch.is_tensor(o) else np.asarray(o) for o in outs]
+    per_len = {}
+    for o in outs:
+        per_len[o.shape[0]] = per_len.get(o.shape[0], 0) + int(np.prod(o.shape[1:]))
+    kept = {n: np.arange(n) if whole else sample_rows(n, e) for n, e in per_len.items()}
+    rows = [kept[o.shape[0]] for o in outs]
+    r = Recorded([o[k] for o, k in zip(outs, rows)], rows, [o.shape for o in outs])
+    os.makedirs(RECORD, exist_ok=True)
+    path = os.path.join(RECORD, fname)
+    recs = _read(path) if os.path.exists(path) else {}
+    recs[name] = [(o.shape, rows[i], r[i]) for i, o in enumerate(outs)]
+    _write(path, recs)
+    return r
 
 
 _lib = None

@@ -52,6 +52,7 @@ def run(monkeypatch, emulated_library):
     monkeypatch.setattr(torch.cuda, "synchronize", lambda *a, **k: None)
     monkeypatch.setattr(torch.cuda, "is_current_stream_capturing", lambda: False)
     monkeypatch.setattr(ref_kernels, "available", lambda: False)
+    monkeypatch.setattr(ref_kernels, "comparing", lambda: False)
 
     def call(module, test, *args, **kwargs):
         mod = importlib.import_module(module)

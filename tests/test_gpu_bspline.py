@@ -1,7 +1,7 @@
 """GPU parity of the B-spline knot -> state kernels and their adjoint (SURVEY.md 8f rank 1), called through the C ABI
 (curobo_b200.backends.trajectory), against
   * the numpy oracle (oracle/bspline_oracle.py), and
-  * the REFERENCE's own kernels compiled from /root/reference into oracle/_ref (same nvcc flags): forward and adjoint
+  * the REFERENCE's own kernels (same nvcc flags; their outputs on these inputs recorded on a B200, tests/ref_kernels.py): forward and adjoint
     are expected to agree to float rounding of identically ordered arithmetic -> tolerance 2 ulp-ish (rtol 1e-6),
     and bit-exact for the adjoint with power-of-two interpolation steps where the summation order is reproduced.
 Tolerances vs the oracle (numpy divides exactly, the kernels use --prec-div=false): rel 2e-5 of the output scale.
@@ -37,6 +37,12 @@ def dev_case(c):
     return d
 
 
+def time_major(outs):
+    """[B,T,D] states -> [T,B,D] (few seeds, many waypoints: the recorded sample keeps whole waypoints, first and last
+    included), the per-seed dt as it is."""
+    return [o.transpose(0, 1) for o in outs[:4]] + list(outs[4:])
+
+
 def ours_forward(c):
     B, Tn, D = c["B"], c["T"], c["D"]
     outs = [torch.full((B, Tn, D), float("nan"), device=DEV) for _ in range(4)]
@@ -65,13 +71,13 @@ def test_forward_vs_oracle_and_reference(kw):
         assert np.isfinite(g).all()
         assert np.allclose(g, w, rtol=2e-5, atol=2e-5 * max(1.0, np.abs(w).max())), f"derivative {k} vs oracle"
     assert np.array_equal(got[4].cpu().numpy(), want[4])
-    if ref_kernels.available():
-        ref = ref_kernels.bspline_forward(c["knots_t"], c["start_t"], c["goal_t"], c["sidx_t"], c["gidx_t"], c["dt_t"],
-                                          c["imp_t"], c["T"], c["degree"])
+    if ref_kernels.comparing():
+        ref = ref_kernels.recorded(("bspline", "forward", case_id(kw)), lambda: time_major(ref_kernels.bspline_forward(
+            c["knots_t"], c["start_t"], c["goal_t"], c["sidx_t"], c["gidx_t"], c["dt_t"], c["imp_t"], c["T"], c["degree"])))
         for k in range(4):
-            g, r = got[k].cpu().numpy(), ref[k].cpu().numpy()
+            g, r = ref.at(k, got[k].cpu().numpy().swapaxes(0, 1)), ref[k]
             assert np.allclose(g, r, rtol=1e-6, atol=1e-6 * max(1.0, np.abs(r).max())), f"derivative {k} vs reference"
-        assert torch.equal(got[4], ref[4])
+        assert np.array_equal(ref.at(4, got[4].cpu().numpy()), ref[4])
 
 
 @pytest.mark.parametrize("kw", CASES, ids=case_id)
@@ -81,10 +87,11 @@ def test_backward_vs_oracle_and_reference(kw):
     want = bo.bspline_backward(*c["grads"], c["traj_dt"], c["goal_idx"], c["implicit"], c["nk"], c["degree"])
     assert np.allclose(got, want, rtol=1e-4, atol=1e-5 * np.abs(want).max())
     steps = c["steps"]
-    if ref_kernels.available() and (steps & (steps - 1)) == 0:
+    if ref_kernels.comparing() and (steps & (steps - 1)) == 0:
         # the reference's shuffle tree is only valid for power-of-two step counts (it mis-pairs lanes otherwise)
-        ref = ref_kernels.bspline_backward(c["grads_t"], c["dt_t"], c["gidx_t"], c["imp_t"], c["nk"], c["degree"]).cpu().numpy()
-        assert np.allclose(got, ref, rtol=1e-6, atol=1e-6 * np.abs(ref).max())
+        ref = ref_kernels.recorded(("bspline", "backward", case_id(kw)), lambda: ref_kernels.bspline_backward(
+            c["grads_t"], c["dt_t"], c["gidx_t"], c["imp_t"], c["nk"], c["degree"]))
+        assert np.allclose(ref.at(0, got), ref[0], rtol=1e-6, atol=1e-6 * np.abs(ref[0]).max())
 
 
 def test_single_dt_vs_oracle_and_reference():
@@ -101,11 +108,12 @@ def test_single_dt_vs_oracle_and_reference():
     got = [out.position, out.velocity, out.acceleration, out.jerk]
     for g, w in zip(got, want[:4]):
         assert np.allclose(g.cpu().numpy(), w, rtol=2e-5, atol=2e-5 * max(1.0, np.abs(w).max()))
-    if ref_kernels.available():
-        ref = ref_kernels.bspline_single_dt(c["knots_t"], c["start_t"], c["goal_t"], c["sidx_t"], c["gidx_t"], idt, c["imp_t"],
-                                            T(interp_h), Tn, 4)
-        for g, r in zip(got, ref[:4]):
-            assert np.allclose(g.cpu().numpy(), r.cpu().numpy(), rtol=1e-6, atol=1e-6 * max(1.0, float(r.abs().max())))
+    if ref_kernels.comparing():
+        ref = ref_kernels.recorded(("bspline", "single_dt"), lambda: time_major(ref_kernels.bspline_single_dt(
+            c["knots_t"], c["start_t"], c["goal_t"], c["sidx_t"], c["gidx_t"], idt, c["imp_t"], T(interp_h), Tn, 4)))
+        for k, g in enumerate(got):
+            r = ref[k]
+            assert np.allclose(ref.at(k, g.cpu().numpy().swapaxes(0, 1)), r, rtol=1e-6, atol=1e-6 * max(1.0, float(np.abs(r).max())))
 
 
 @pytest.mark.parametrize("implicit", [False, True])

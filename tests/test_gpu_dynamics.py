@@ -1,6 +1,6 @@
 """GPU parity of the RNEA inverse-dynamics kernels (SURVEY.md 8f rank 3) through the C ABI
-(curobo_b200.backends.dynamics) against the numpy oracle and the REFERENCE's own kernels compiled into oracle/_ref
-(serial threads_per_batch = 1 path: same order of every sum -> expected equal to float rounding, rtol 1e-5)."""
+(curobo_b200.backends.dynamics) against the numpy oracle and the REFERENCE's own kernels (outputs recorded on a B200,
+tests/ref_kernels.py; serial threads_per_batch = 1 path: same order of every sum -> expected equal to float rounding, rtol 1e-5)."""
 import numpy as np
 import pytest
 import torch
@@ -50,18 +50,22 @@ def test_rnea_vs_oracle_and_reference(robot, B, seed):
         want = do.rnea_backward(c["grad_tau"], c["q"], c["qd"], cache_w, *m)
         for g, w, n in zip((gq, gqd, gqdd), want, ("grad_q", "grad_qd", "grad_qdd")):
             close(g.cpu().numpy(), w, 3e-4, n + " vs oracle")
-    if ref_kernels.available():
-        rt, rc = ref_kernels.rnea_forward(model, q, qd, qdd, nl, D, nlev)
-        rg = ref_kernels.rnea_backward(model, gt, q, qd, rc, nl, D, nlev)
-        torch.cuda.synchronize()
-        close(tau.cpu().numpy(), rt.cpu().numpy(), 1e-5, "tau vs reference")
-        close(cache.cpu().numpy().reshape(B, nl, 20)[:, :, :18], rc.cpu().numpy().reshape(B, nl, 20)[:, :, :18], 1e-5, "cache vs reference")
-        for g, r, n in zip((gq, gqd, gqdd), rg, ("grad_q", "grad_qd", "grad_qdd")):
-            close(g.cpu().numpy(), r.cpu().numpy(), 2e-5, n + " vs reference")
-        # caches are interchangeable: our adjoint on the reference's cache
-        g2 = [torch.zeros((B, D), device=DEV) for _ in range(3)]
-        dynamics_cu.launch_rnea_backward(*g2, gt, q, qd, *model, rc, B, nl, D, nlev)
-        close(g2[0].cpu().numpy(), rg[0].cpu().numpy(), 2e-5, "adjoint on the reference cache")
+    if ref_kernels.comparing():
+        def reference():
+            rt, rc = ref_kernels.rnea_forward(model, q, qd, qdd, nl, D, nlev)
+            return [rt, rc] + ref_kernels.rnea_backward(model, gt, q, qd, rc, nl, D, nlev)
+        r = ref_kernels.recorded(("dynamics", "rnea", robot, B, seed), reference)
+        close(r.at(0, tau.cpu().numpy()), r[0], 1e-5, "tau vs reference")
+        close(r.at(1, cache.cpu().numpy()).reshape(-1, nl, 20)[:, :, :18], r[1].reshape(-1, nl, 20)[:, :, :18], 1e-5,
+              "cache vs reference")
+        for i, (g, n) in enumerate(zip((gq, gqd, gqdd), ("grad_q", "grad_qd", "grad_qdd"))):
+            close(r.at(2 + i, g.cpu().numpy()), r[2 + i], 2e-5, n + " vs reference")
+        # caches are interchangeable: our adjoint on the reference's cache (its recorded rows, the same rows as grad_q's)
+        ir = torch.as_tensor(r.rows(1), device=DEV)
+        g2 = [torch.zeros((len(ir), D), device=DEV) for _ in range(3)]
+        dynamics_cu.launch_rnea_backward(*g2, gt[ir].contiguous(), q[ir].contiguous(), qd[ir].contiguous(), *model,
+                                         T(r[1]), len(ir), nl, D, nlev)
+        close(g2[0].cpu().numpy(), r[2], 2e-5, "adjoint on the reference cache")
 
 
 def test_dynamics_operator_autograd_and_graph():

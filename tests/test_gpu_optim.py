@@ -1,6 +1,6 @@
 """GPU parity of the optimizer-side kernels (SURVEY.md 8f rank 2) through the C ABI
-(curobo_b200.backends.optimization) against the numpy oracle and the REFERENCE's own kernels compiled into
-oracle/_ref, and the whole loop (L-BFGS step -> fused rollout -> line search) solving real problems.
+(curobo_b200.backends.optimization) against the numpy oracle and the REFERENCE's own kernels (their outputs recorded on a
+B200, tests/ref_kernels.py), and the whole loop (L-BFGS step -> fused rollout -> line search) solving real problems.
 
 Sums are associated like the reference's block reductions, so float results are expected bit-equal to the reference
 kernels; the tests assert rtol 1e-6 and report exact equality where it must hold (copies, indices, counters).
@@ -55,15 +55,20 @@ def test_lbfgs_step_vs_oracle_and_reference(kw):
     # parity target.  Its global-memory fallback disagrees with it by 10-50 % and is not even run-to-run deterministic
     # for v_dim > 32 (measured on B200: scripts/debug_lbfgs.py), so it is only compared for single-warp problems.
     variants = ([True] if fits_shared else []) + ([False] if V <= 32 else [])
-    if ref_kernels.available() and m in (3, 5, 7, 15, 27, 31):
-        for shared in variants:
+    if ref_kernels.comparing() and m in (3, 5, 7, 15, 27, 31):
+        ours = [a.cpu().numpy() for a in (step, t["rho"], t["Y"], t["S"], t["x_0"])]
+
+        def reference(shared):
             r = {k: T(v) for k, v in c.items()}
             rstep = torch.zeros_like(step)
             ref_kernels.lbfgs_step(rstep, r["rho"], r["Y"], r["S"], r["q"], r["x_0"], r["grad_0"], r["grad_q"], 0.01, True, shared)
-            torch.cuda.synchronize()
-            assert torch.equal(t["Y"], r["Y"]) and torch.equal(t["S"], r["S"]) and torch.equal(t["x_0"], r["x_0"])
-            close(t["rho"].cpu().numpy(), r["rho"].cpu().numpy(), 1e-6)
-            close(step.cpu().numpy(), rstep.cpu().numpy(), 1e-6)
+            return rstep, r["rho"], r["Y"], r["S"], r["x_0"]
+        for shared in variants:
+            ref = ref_kernels.recorded(("optim", "lbfgs_step", lbfgs_id(kw), shared), lambda: reference(shared))
+            o_step, o_rho, o_Y, o_S, o_x0 = (ref.at(i, a) for i, a in enumerate(ours))
+            assert np.array_equal(o_Y, ref[2]) and np.array_equal(o_S, ref[3]) and np.array_equal(o_x0, ref[4])
+            close(o_rho, ref[1], 1e-6)
+            close(o_step, ref[0], 1e-6)
 
 
 def test_lbfgs_autograd_function_and_search_points():
@@ -122,12 +127,13 @@ def test_line_search_vs_oracle_and_reference(kw, strong, approx):
     for k in ("selected_cost", "selected_action", "selected_gradient", "exploration_cost", "exploration_action",
               "exploration_gradient", "best_cost", "best_action", "best_iteration", "current_iteration", "converged"):
         assert np.array_equal(got[k], o[k]), k
-    if ref_kernels.available() and V >= n:      # the reference kernel needs opt_dim >= n_linesearch threads
-        rs = ls_state(c, B, n, V)
-        ref_kernels.line_search(rs, sc, sa, sg, sd, mg, 1e-5, 0.9, strong, approx)
-        torch.cuda.synchronize()
-        for k in st:
-            assert torch.equal(st[k], rs[k]), k
+    if ref_kernels.comparing() and V >= n:      # the reference kernel needs opt_dim >= n_linesearch threads
+        def reference():
+            rs = ref_kernels.line_search(ls_state(c, B, n, V), sc, sa, sg, sd, mg, 1e-5, 0.9, strong, approx)
+            return [rs[k] for k in st]
+        ref = ref_kernels.recorded(("optim", "line_search", ls_id(kw), strong, approx), reference)
+        for i, k in enumerate(st):
+            assert np.array_equal(ref.at(i, got[k]), ref[i]), k
 
 
 def test_lbfgs_opt_solves_quadratics():

@@ -57,16 +57,15 @@ def test_fk_forward_vs_oracle_and_reference(robot, n):
     np.testing.assert_allclose(st.tool_pose_position.cpu().numpy().reshape(pos.shape), pos, atol=1e-5)
     quat_close(st.tool_pose_quaternion.cpu().numpy().reshape(quat.shape), quat, 1e-5)
     assert (st.tool_pose_quaternion[..., 0] >= 0).all()
-    if ref_kernels.available():
-        rp, rq, rs, rc = ref_kernels.fk_forward(kin.params, T(q))
-        torch.cuda.synchronize()
+    if ref_kernels.comparing():
+        r = ref_kernels.recorded(("parity", "fk_forward", robot, n), lambda: ref_kernels.fk_forward(kin.params, T(q)))
         # our kernel vs the reference kernel, and (pinning the oracle) oracle vs the reference kernel
-        np.testing.assert_allclose(st.cumul_mat.cpu().numpy().reshape(cum.shape), rc.cpu().numpy(), atol=1e-5)
-        np.testing.assert_allclose(st.robot_spheres.cpu().numpy().reshape(sph.shape), rs.cpu().numpy(), atol=1e-5)
-        np.testing.assert_allclose(rc.cpu().numpy(), cum, atol=1e-5)
-        np.testing.assert_allclose(rs.cpu().numpy(), sph, atol=1e-5)
-        np.testing.assert_allclose(rp.cpu().numpy(), pos, atol=1e-5)
-        quat_close(rq.cpu().numpy(), quat, 1e-5)
+        np.testing.assert_allclose(r.at(3, st.cumul_mat.cpu().numpy().reshape(cum.shape)), r[3], atol=1e-5)
+        np.testing.assert_allclose(r.at(2, st.robot_spheres.cpu().numpy().reshape(sph.shape)), r[2], atol=1e-5)
+        np.testing.assert_allclose(r[3], r.at(3, cum), atol=1e-5)
+        np.testing.assert_allclose(r[2], r.at(2, sph), atol=1e-5)
+        np.testing.assert_allclose(r[0], r.at(0, pos), atol=1e-5)
+        quat_close(r[1], r.at(1, quat), 1e-5)
 
 
 def test_fk_without_spheres_entry_point():
@@ -137,10 +136,11 @@ def test_fk_backward_vs_oracle_and_reference(robot, n, sparse):
     loss.backward()
     got = qt.grad.cpu().numpy()
     grad_close(got, want)
-    if ref_kernels.available():
-        ref = ref_kernels.fk_backward(kin.params, T(cum), T(gp), T(gq), T(gs)).cpu().numpy()
-        grad_close(got, ref)
-        grad_close(want, ref)          # pins the oracle's backward
+    if ref_kernels.comparing():
+        r = ref_kernels.recorded(("parity", "fk_backward", robot, n, sparse),
+                                 lambda: ref_kernels.fk_backward(kin.params, T(cum), T(gp), T(gq), T(gs)))
+        grad_close(r.at(0, got), r[0])
+        grad_close(r.at(0, want), r[0])          # pins the oracle's backward
 
 
 def test_fk_backward_mimic_and_negative_axis():
@@ -199,11 +199,14 @@ def test_self_collision_vs_oracle_and_reference(robot, n):
     grad_close(got_g, want_g)
     d.sum().backward()
     grad_close(st.grad.cpu().numpy().reshape(want_g.shape), want_g)
-    if ref_kernels.available():
-        rd, rv = ref_kernels.self_collision(rm, T(sph.reshape(n, 1, -1, 4)), cost.sphere_padding, cost.pairs, 5000.0)
-        np.testing.assert_allclose(got_c, rd.cpu().numpy().reshape(n), rtol=1e-4, atol=1e-6 * want_c.max())
-        grad_close(got_g, rv.cpu().numpy().reshape(want_g.shape))
-        np.testing.assert_allclose(want_c, rd.cpu().numpy().reshape(n), rtol=1e-4, atol=1e-6 * want_c.max())
+    if ref_kernels.comparing():
+        def reference():
+            d, v = ref_kernels.self_collision(rm, T(sph.reshape(n, 1, -1, 4)), cost.sphere_padding, cost.pairs, 5000.0)
+            return d.view(n), v.view(want_g.shape)
+        r = ref_kernels.recorded(("parity", "self_collision", robot, n), reference, whole=True)   # sparse: every row
+        np.testing.assert_allclose(r.at(0, got_c), r[0], rtol=1e-4, atol=1e-6 * want_c.max())
+        grad_close(r.at(1, got_g), r[1])
+        np.testing.assert_allclose(r.at(0, want_c), r[0], rtol=1e-4, atol=1e-6 * want_c.max())
 
 
 def test_self_collision_lazy_zeroing_and_golden():

@@ -1,6 +1,6 @@
 """GPU parity of the exact nearest-site transform (SURVEY.md 8f rank 4) through the C ABI (curobo_b200.backends.pba /
-curobo_b200.esdf.ParallelBandingEDT) against scipy's exact EDT, the oracle and the REFERENCE's own PBA+ kernels compiled into
-oracle/_ref.  Integer work: the squared distance to the reported site must be bit exact and the reported site must be a site
+curobo_b200.esdf.ParallelBandingEDT) against scipy's exact EDT, the oracle and the REFERENCE's own PBA+ kernels (their outputs
+recorded on a B200, tests/ref_kernels.py).  Integer work: the squared distance to the reported site must be bit exact and the reported site must be a site
 (which of several equidistant sites is reported is unspecified in the reference too).  Written after this round's GPU budget
 was spent: first run on a B200 in round 2 (banded schedule)."""
 import numpy as np
@@ -52,10 +52,12 @@ def test_nearest_site_transform_is_exact(kind, shape, p):
     want = E.unsigned_distance_fp16(sites.cpu().numpy(), 0.02)
     assert np.abs(dist.astype(np.float32) - want.astype(np.float32)).max() <= 2e-3 * max(1.0, float(want.astype(np.float32).max()))
     assert (dist[occ] == 0).all() if occ.any() else (dist == np.float16(1e4)).all()
-    if ref_kernels.available() and min(shape) >= 4:  # the reference is only ever run on genuinely 3-D grids
-        ref = ref_kernels.pba3d(seed_sites_from_occupancy(torch.as_tensor(occ).to(DEV)))
-        torch.cuda.synchronize()
-        rd2 = E.squared_distance(ref.cpu().numpy())
+    if ref_kernels.comparing() and min(shape) >= 4:  # the reference is only ever run on genuinely 3-D grids
+        def reference():
+            ref = ref_kernels.pba3d(seed_sites_from_occupancy(torch.as_tensor(occ).to(DEV)))
+            return E.squared_distance(ref.cpu().numpy()).astype(np.int32).reshape(-1, shape[2])    # rows = z columns
+        r = ref_kernels.recorded(("edt", "pba3d", kind, *shape, p), reference)
+        d2, rd2 = r.at(0, d2.reshape(-1, shape[2])), r[0]
         if not np.array_equal(d2, rd2):
             # our result is already proven exact against scipy above; the launcher of the reference kernels (oracle/_ref) has
             # never run on a GPU, so a mismatch here is reported without stopping the first GPU pass -- make it an assert once

@@ -67,12 +67,14 @@ def test_center_of_mass_and_its_gradient(robot, n):
     st0 = Kinematics(rm, DEV).compute_kinematics(T(q))
     assert st0.center_of_mass is None and torch.equal(st0.robot_spheres, st.robot_spheres.detach())
     import ref_kernels
-    if ref_kernels.available():      # the reference's own kernels, COMPUTE_COM = true (launcher never run on a GPU yet: soft)
-        rs, rc, rcom = ref_kernels.fk_forward_com(kin.params, T(q))
-        torch.cuda.synchronize()
-        zp = torch.zeros((n, rm.num_tool_frames, 3), device=DEV)
-        zq = torch.zeros((n, rm.num_tool_frames, 4), device=DEV)
-        rg = ref_kernels.fk_backward_com(kin.params, rc, rcom, zp, zq, T(gs).view(n, -1, 4).contiguous(), T(g)).cpu().numpy()
-        ok = np.allclose(got, rcom.cpu().numpy(), rtol=1e-5, atol=2e-6) and np.allclose(got_g, rg, rtol=2e-3, atol=2e-5 * np.abs(rg).max())
+    if ref_kernels.comparing():      # the reference's own kernels, COMPUTE_COM = true (launcher never run on a GPU yet: soft)
+        def reference():
+            rs, rc, rcom = ref_kernels.fk_forward_com(kin.params, T(q))
+            zp = torch.zeros((n, rm.num_tool_frames, 3), device=DEV)
+            zq = torch.zeros((n, rm.num_tool_frames, 4), device=DEV)
+            return rcom, ref_kernels.fk_backward_com(kin.params, rc, rcom, zp, zq, T(gs).view(n, -1, 4).contiguous(), T(g))
+        r = ref_kernels.recorded(("com", "fk_com", robot, n), reference)
+        ok = np.allclose(r.at(0, got), r[0], rtol=1e-5, atol=2e-6) and \
+            np.allclose(r.at(1, got_g), r[1], rtol=2e-3, atol=2e-5 * np.abs(r[1]).max())
         if not ok:
             pytest.xfail("differs from the reference's COMPUTE_COM kernels (reference launcher unvalidated on a GPU)")
